@@ -1,6 +1,6 @@
 """bench.py -- Envelope-Q gradient updates/sec on synthetic transitions (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one gradient update of Envelope Q-learning (reference envelope.py:269-334, gradient_updates=1) at
@@ -22,6 +22,10 @@ grad clip -> Adam (+ target sync every 200 steps).
                  a bounded NUMBER of updates (not a bounded batch); cpu_dedup_restatement: the de-duplicated CPU restatement for context.
 N > 1: every rank runs an independent update stream (weak scaling, no data-path collective); the ranks exchange their non-dominated
 fronts with ONE NCCL all-gather per evaluation round, which is timed separately (config.ms_eval_round_*), not inside the updates.
+
+--dump-outputs DIR (envelope workload): after the timed updates, rank 0 writes what the last update of each arm handed its caller -- loss,
+sampled replay indices, written-back priorities and the updated online Q-network -- as DIR/<name>.npy (float32 / float64; `e2e.` prefix for
+the host-replay arm).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -116,6 +120,24 @@ def _make_agent(dev, seed, on_device):
     env = FakeEnv(obs_dim=OBS, n_actions=A, reward_dim=D)
     return Envelope(env, batch_size=B, num_sample_w=W, per=True, buffer_size=STORE, net_arch=NET, log=False, seed=seed, device=dev,
                     replay_on_device=on_device)
+
+
+def _last_update_outputs(agent, prefix=""):
+    """What Envelope.update() hands its caller after its last gradient step, as host arrays: the critic loss, the replay indices it sampled
+    (float64: exact), the priorities it wrote back and the updated online Q-network."""
+    out = {prefix + "loss": np.array([agent.last_loss_host()], np.float32), prefix + "indices": np.asarray(agent._last_inds, np.float64),
+           prefix + "priorities": np.asarray(agent._last_priority, np.float32)}
+    for name, p in agent.q_net.named_parameters():
+        out[f"{prefix}q_net.{name}"] = p.detach().float().cpu().numpy()
+    return out
+
+
+def _dump_outputs(path, arrays):
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "dumped outputs exceed 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def time_envelope_kernel(dev, replays=25):
@@ -455,6 +477,7 @@ def run_b200(args, rank, local_rank, world):
     K, Wm = args.steps, args.warmup
     store = synthetic_store(STORE, OBS, A, D, seed=0)
     np.random.seed(1000 + rank)
+    th.manual_seed(rank)  # network initialisation: torch's default generator is not seeded reproducibly
 
     # ---------------- `value`: the full update of SURVEY 8(d) -- PER sample + targets + forward/backward + optimiser + priority write-back --
     # through the public API with the replay store RESIDENT IN HBM: per step the host walks the sum-tree, 9 KB of indices + weights go
@@ -500,6 +523,7 @@ def run_b200(args, rank, local_rank, world):
     th.cuda.synchronize()
     ms_steps = e0.elapsed_time(em)
     clocks = sampler.result()
+    outputs = _last_update_outputs(agent) if args.dump_outputs and rank == 0 else None
     gpu_launches = (ops.launch_count - launches0) + launches_per_step * K
     # the evaluation round, timed on its own (it is NOT part of an update): 3 rounds, the last one reported
     for _ in range(3):
@@ -542,6 +566,9 @@ def run_b200(args, rank, local_rank, world):
     e2e_value = world * K / (float(t2.item()) * 1e-3)
     h2d = B * (OBS * 4 * 2 + 4 + D * 4 + 4) + W * D * 4
     d2h = B * 4 + 4
+    if args.dump_outputs and rank == 0:
+        outputs.update(_last_update_outputs(agent_h, "e2e."))
+        _dump_outputs(args.dump_outputs, outputs)
 
     if rank != 0:
         if world > 1:
@@ -822,7 +849,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="envelope", choices=["envelope", "morld", "envelope_dp"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed update as DIR/<name>.npy (envelope workload, rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "envelope"):
+        ap.error("--dump-outputs is available for --impl b200 --workload envelope")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -8,10 +8,9 @@ It registers empty stand-in modules in ``sys.modules`` carrying only the *names*
 touches at import time (SURVEY.md Appendix B), and offers a ``FakeEnv`` exposing the attributes
 ``MOAgent.extract_env_info`` reads (reference ``morl_baselines/common/morl_algorithm.py:248-273``).
 
-Only ``tests/golden/make_golden.py`` (fixture generation, run in the build container), the
-``-m "not gpu"`` differential tests that are skipped when /root/reference is absent, and
-``bench.py --impl reference`` (when the mount exists) may use this module.  /root/reference does
-not exist on the GPU box: everything here degrades to ``reference_available() == False`` there.
+Only the golden-data generators under ``tests/golden/`` and ``bench.py`` (its CPU arm, when the
+reference is present) may use this module; the tests compare against the stored golden data and
+never import the reference.  Without the reference, ``reference_available()`` is False.
 """
 
 from __future__ import annotations
