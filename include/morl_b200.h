@@ -387,6 +387,25 @@ MORL_API size_t morl_gemm_mn_workspace_bytes(int M, int a_cols, int b_cols);
 MORL_API int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long g_plane_stride, int ldg, int g_cols, const float* g_scale,
                                      const void* h_planes, long long h_plane_stride, int ldh, int h_cols, const float* h_scale, int M,
                                      int transpose_out, float* out, int ld_out, float* colsum_out, void* workspace, void* stream);
+/* Up to MORL_MN_MAX_JOBS weight-gradient products over the same M rows in ONE persistent launch plus ONE reduction launch: job j computes
+ * out[n, k] (and colsum_out[n]) exactly as morl_gemm_planes_mn_f32 with transpose_out = 0 does -- bit-identical -- but the operand stream does
+ * not stop between the products (the backward pass of an update: the output layer and every hidden layer).  Per job: ldg, ldh multiples of
+ * 64, ldh <= 256, h_cols % 4 == 0, ld_out % 4 == 0, out 16-byte aligned (others are refused with MORL_ERR_UNSUPPORTED); colsum_out nullable.
+ *   workspace: morl_gemm_mn_multi_workspace_bytes(jobs, n_jobs, M) bytes, 16-byte aligned. */
+#define MORL_MN_MAX_JOBS 4
+typedef struct MorlMnJob {
+    const void* g_planes;      /* [P][M][ldg], scaled by *g_scale (NULL = 1) */
+    long long g_plane_stride;  /* elements between planes */
+    const float* g_scale;
+    const void* h_planes;      /* [P][M][ldh], scaled by *h_scale (NULL = 1) */
+    long long h_plane_stride;
+    const float* h_scale;
+    float* out;                /* [g_cols][ld_out] */
+    float* colsum_out;         /* [g_cols] or NULL */
+    int ldg, g_cols, ldh, h_cols, ld_out;
+} MorlMnJob;
+MORL_API size_t morl_gemm_mn_multi_workspace_bytes(const MorlMnJob* jobs, int n_jobs, int M);
+MORL_API int morl_gemm_planes_mn_multi_f32(int fmt, const MorlMnJob* jobs, int n_jobs, int M, void* workspace, void* stream);
 /* out[n] = (1 / *scale) sum_m sum_p planes[p][m][n]  (bias gradients); workspace: 296 * N floats */
 MORL_API int morl_colsum_planes(int fmt, const void* planes, long long plane_stride, const float* scale, int M, int ld, int N, float* out,
                                 void* workspace, void* stream);

@@ -69,6 +69,8 @@ SIGNATURES = {
     "morl_pairs_relu_split_planes": (_i, [_i, _vp, _vp, _i, _i, _i, _vp, C.c_longlong, _vp, _vp, _vp]),
     "morl_gemm_mn_workspace_bytes": (_sz, [_i, _i, _i]),
     "morl_gemm_planes_mn_f32": (_i, [_i, _vp, C.c_longlong, _i, _i, _vp, _vp, C.c_longlong, _i, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp]),
+    "morl_gemm_mn_multi_workspace_bytes": (_sz, [_vp, _i, _i]),
+    "morl_gemm_planes_mn_multi_f32": (_i, [_i, _vp, _i, _i, _vp, _vp]),
     "morl_colsum_planes": (_i, [_i, _vp, C.c_longlong, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "morl_pairs_grad_reduce_planes": (_i, [_i, _vp, C.c_longlong, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "morl_pair_layer1_uv_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
@@ -86,6 +88,16 @@ class SplitJob(C.Structure):
 
     _fields_ = [("src", _vp), ("dst_planes", _vp), ("plane_stride", C.c_longlong), ("scale", _vp), ("rows", _i), ("cols", _i), ("ld_src", _i),
                 ("transpose", _i), ("rows_pad", _i), ("ldp", _i), ("auto_scale", _i), ("target_exp", _i)]
+
+
+MN_MAX_JOBS = 4
+
+
+class MnJob(C.Structure):
+    """MorlMnJob of include/morl_b200.h"""
+
+    _fields_ = [("g_planes", _vp), ("g_plane_stride", C.c_longlong), ("g_scale", _vp), ("h_planes", _vp), ("h_plane_stride", C.c_longlong),
+                ("h_scale", _vp), ("out", _vp), ("colsum_out", _vp), ("ldg", _i), ("g_cols", _i), ("ldh", _i), ("h_cols", _i), ("ld_out", _i)]
 
 
 _lib = None

@@ -995,6 +995,218 @@ gemm_planes_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     }
 }
 
+// shared memory of the MN-major kernels: the TMA ring (A: 2 chunks, B: up to 4 chunks per stage), barriers, the 4 KB tile of ones, slack
+template <int FMT>
+constexpr size_t mn_smem_bytes() {
+    return (size_t)PlaneFmt<FMT>::kStagesMn * (6u * PlaneFmt<FMT>::P * kMnKT * 128u) + 256 + 1024 + 64 + 1024 + 4096;
+}
+
+// -----------------------------------------------------------------------------------------------------------------
+// Several weight-gradient products  dW_j = G_j^T H_j (+ db_j = colsum(G_j))  in ONE persistent launch (the backward pass of an update:
+// the output layer and every hidden layer).  A unit is (job, column tile, split) with exactly the split boundaries, MMA shape and MMA issue
+// order of gemm_planes_mn_kernel, so every partial is bit-identical to the per-layer launch; units are dealt round-robin to the CTAs.  What
+// the launch gains is continuity: the TMA ring streams the next unit's operands while the current unit's MMAs and epilogue run, and the
+// prologue (barriers, TMEM allocation, tile of ones) is paid once instead of once per layer.
+// The accumulator (256 + 16 columns) cannot be double-buffered in 512 TMEM columns: the 8 epilogue warps copy it to registers (two warps per
+// lane quadrant, half of the columns each), release it, and store the partials while the MMAs of the next unit already run.
+// Only the real rows (n < g_cols) of a tile are stored: partials are [S][g_cols][NB].
+// -----------------------------------------------------------------------------------------------------------------
+constexpr int kMnMaxJobs = MORL_MN_MAX_JOBS;
+
+struct MnJobArgs {
+    int n_tiles, NB, rows_per_split, S;  // as GemmMnArgs
+    int g_cols, h_cols, ld_out;
+    int unit0;                           // first unit of the job in the launch's unit sequence
+    int red_block0, red_main_blocks;     // reduction launch: first block of the job; blocks of the matrix part (column-sum blocks follow)
+    float* partial;                      // [S][g_cols][NB]
+    float* colsum_partial;               // [S][g_cols] or nullptr
+    float* out;                          // [g_cols][ld_out]
+    float* colsum_out;                   // [g_cols] or nullptr
+    const float* g_scale;
+    const float* h_scale;
+};
+
+struct alignas(64) MnMulti {
+    CUtensorMap tmA[kMnMaxJobs], tmB[kMnMaxJobs];  // G_j (A = G^T) and H_j (B = H^T), make_plane_map_mn
+    MnJobArgs job[kMnMaxJobs];
+    int n_jobs, n_units, M;
+};
+
+template <int FMT>
+__global__ void __launch_bounds__(kGemmThreads, 1) gemm_planes_mn_multi_kernel(const __grid_constant__ MnMulti mj) {
+    using F = PlaneFmt<FMT>;
+    constexpr int P = F::P;
+    constexpr int kStages = F::kStagesMn;
+    extern __shared__ uint8_t gsmem_raw[];
+    uint8_t* gsmem = gsmem_raw + ((1024u - (g_smem_u32(gsmem_raw) & 1023u)) & 1023u);
+    constexpr uint32_t chunk_bytes = (uint32_t)P * kMnKT * 128u;
+    constexpr uint32_t a_stage = 2u * chunk_bytes;
+    constexpr uint32_t b_stage = 4u * chunk_bytes;
+    uint8_t* smA = gsmem;
+    uint8_t* smB = gsmem + kStages * a_stage;
+    uint64_t* full = reinterpret_cast<uint64_t*>(smB + kStages * b_stage);
+    uint64_t* empty = full + kStages;
+    uint64_t* tfull = empty + kStages;  // accumulator complete (MMA commit)
+    uint64_t* tempty = tfull + 1;       // accumulator copied to registers (8 epilogue warps)
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 1);
+    uint8_t* ones_b = reinterpret_cast<uint8_t*>(tmem_slot + 4);
+    uint32_t* ones = reinterpret_cast<uint32_t*>(ones_b + ((1024u - (g_smem_u32(ones_b) & 1023u)) & 1023u));
+    for (int t = threadIdx.x; t < 1024; t += blockDim.x) ones[t] = F::kOnes2;
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    auto job_of = [&](int u) {
+        int j = 0;
+        while (j + 1 < mj.n_jobs && u >= mj.job[j + 1].unit0) ++j;
+        return j;
+    };
+    // unit u -> job j, column tile nt, split (numbered like the blocks of gemm_planes_mn_kernel) and its row range
+    auto unit_of = [&](int u, int& j, int& nt, int& split, int& m_begin, int& n_kblk) {
+        j = job_of(u);
+        const MnJobArgs& jb = mj.job[j];
+        const int l = u - jb.unit0;
+        nt = l % jb.n_tiles;
+        split = l / jb.n_tiles;
+        m_begin = split * jb.rows_per_split;
+        const int m_end = min(mj.M, m_begin + jb.rows_per_split);
+        n_kblk = (m_end - m_begin + kMnKT - 1) / kMnKT;  // >= 1: the host sizes S so that no split is empty
+    };
+
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < kStages; ++s) {
+            g_mbar_init(&full[s], 1);
+            g_mbar_init(&empty[s], 1);
+        }
+        g_mbar_init(tfull, 1);
+        g_mbar_init(tempty, 8);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(g_smem_u32(tmem_slot)) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    pdl_enter();  // (nothing above touches global memory)
+
+    if (warp == 0) {
+        if (lane == 0) {
+            uint32_t stage = 0, phase = 0;  // one ring across all units of the CTA
+            for (int u = blockIdx.x; u < mj.n_units; u += gridDim.x) {
+                int j, nt, split, m_begin, n_kblk;
+                unit_of(u, j, nt, split, m_begin, n_kblk);
+                const CUtensorMap* tmA = &mj.tmA[j];
+                const CUtensorMap* tmB = &mj.tmB[j];
+                const int nb_chunks = mj.job[j].NB / 64;
+                for (int kb = 0; kb < n_kblk; ++kb) {
+                    g_mbar_wait(&empty[stage], phase ^ 1u);
+                    g_mbar_expect_tx(&full[stage], (2u + (uint32_t)nb_chunks) * chunk_bytes);
+                    const int m0 = m_begin + kb * kMnKT;
+                    for (int c = 0; c < 2; ++c) tma_load_3d(smA + stage * a_stage + c * chunk_bytes, tmA, &full[stage], nt * 128 + c * 64, m0, 0);
+                    for (int c = 0; c < nb_chunks; ++c) tma_load_3d(smB + stage * b_stage + c * chunk_bytes, tmB, &full[stage], c * 64, m0, 0);
+                    if (++stage == kStages) {
+                        stage = 0;
+                        phase ^= 1u;
+                    }
+                }
+            }
+        }
+    } else if (warp == 1) {
+        if (lane == 0) {
+            const uint32_t idesc_ones = (1u << 4) | F::kIdescAB | (1u << 15) | (1u << 16) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+            const uint64_t ones_desc = make_desc_mn_sw128(g_smem_u32(ones), chunk_bytes);
+            constexpr uint32_t plane = kMnKT * 128u;
+            uint32_t stage = 0, phase = 0, it = 0;
+            for (int u = blockIdx.x; u < mj.n_units; u += gridDim.x, ++it) {
+                int j, nt, split, m_begin, n_kblk;
+                unit_of(u, j, nt, split, m_begin, n_kblk);
+                const bool colsum = mj.job[j].colsum_partial != nullptr;
+                const uint32_t idesc = (1u << 4) | F::kIdescAB | (1u << 15) | (1u << 16) | ((uint32_t)(mj.job[j].NB >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+                g_mbar_wait(tempty, (it & 1u) ^ 1u);  // the previous unit's accumulator has been copied out
+                tc_fence_after();
+                for (int kb = 0; kb < n_kblk; ++kb) {
+                    g_mbar_wait(&full[stage], phase);
+                    tc_fence_after();
+                    const uint32_t a0 = g_smem_u32(smA + stage * a_stage);
+                    const uint32_t b0 = g_smem_u32(smB + stage * b_stage);
+#pragma unroll
+                    for (int ks = 0; ks < kMnKT / 16; ++ks) {
+#pragma unroll
+                        for (int t = 0; t < F::NPROD; ++t) {
+                            const uint64_t ad = make_desc_mn_sw128(a0 + F::pa(t) * plane + ks * 2048u, chunk_bytes);
+                            const uint64_t bd = make_desc_mn_sw128(b0 + F::pb(t) * plane + ks * 2048u, chunk_bytes);
+                            tc_mma_bf16(tmem_base, ad, bd, idesc, (kb | ks | t) != 0 ? 1u : 0u);
+                        }
+                        if (colsum) {
+#pragma unroll
+                            for (int pl = P - 1; pl >= 0; --pl)
+                                tc_mma_bf16(tmem_base + 256u, make_desc_mn_sw128(a0 + pl * plane + ks * 2048u, chunk_bytes), ones_desc, idesc_ones,
+                                            (kb | ks | (P - 1 - pl)) != 0 ? 1u : 0u);
+                        }
+                    }
+                    tc_commit(&empty[stage]);
+                    if (++stage == kStages) {
+                        stage = 0;
+                        phase ^= 1u;
+                    }
+                }
+                tc_commit(tfull);
+            }
+        }
+    } else {
+        const int quad = warp & 3;
+        const int half = (warp - 2) >> 2;
+        const uint32_t t_row = tmem_base + ((uint32_t)(quad * 32) << 16);
+        uint32_t it = 0;
+        for (int u = blockIdx.x; u < mj.n_units; u += gridDim.x, ++it) {
+            // (only the job is live across the accumulator copy: 128 registers of it leave little room)
+            const int j = job_of(u);
+            const int ncol = mj.job[j].NB >> 1;  // this warp's accumulator columns: [half * ncol, half * ncol + ncol), a multiple of 32
+            const bool colsum = half == 0 && mj.job[j].colsum_partial != nullptr;
+            g_mbar_wait(tfull, it & 1u);
+            tc_fence_after();
+            uint32_t cs = 0;
+            if (colsum) cs = tc_ld1(t_row + 256u);
+            uint32_t v[4][32];
+#pragma unroll
+            for (int c = 0; c < 4; ++c)
+                if (c * 32 < ncol) tc_ld32(t_row + (uint32_t)(half * ncol + c * 32), v[c]);
+            tc_ld_wait();
+            // the values must be in registers before the accumulator is released: tie them to this point
+#pragma unroll
+            for (int c = 0; c < 4; ++c)
+#pragma unroll
+                for (int e = 0; e < 32; ++e) asm volatile("" : "+r"(v[c][e]));
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) g_mbar_arrive(tempty);
+            const MnJobArgs& jb = mj.job[j];
+            const int l = u - jb.unit0, nt = l % jb.n_tiles, split = l / jb.n_tiles;
+            const int row = nt * 128 + quad * 32 + lane;  // output row (n)
+            if (row < jb.g_cols) {
+                float* prow = jb.partial + ((size_t)split * jb.g_cols + row) * jb.NB + half * ncol;
+#pragma unroll
+                for (int c = 0; c < 4; ++c)
+                    if (c * 32 < ncol) {
+#pragma unroll
+                        for (int e = 0; e < 32; e += 4)
+                            *reinterpret_cast<float4*>(prow + c * 32 + e) = make_float4(__uint_as_float(v[c][e]), __uint_as_float(v[c][e + 1]),
+                                                                                         __uint_as_float(v[c][e + 2]), __uint_as_float(v[c][e + 3]));
+                    }
+                if (colsum) jb.colsum_partial[(size_t)split * jb.g_cols + row] = __uint_as_float(cs);
+            }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+    }
+}
+
 // out[r][c] (or out[c][r] if transpose) = mul * sum_s partial[s][r][c] for r < rows, c < cols, mul = 1 / (scale_a * scale_b).
 // blockDim = (32, 8): 32 consecutive output elements per block, the S partials are strided over threadIdx.y (fixed order:
 // deterministic), then combined through shared memory.
@@ -1049,15 +1261,14 @@ __global__ void __launch_bounds__(256) reduce_partials_kernel(const float* __res
 // for the non-transposed case with cols % 4 == 0 -- the weight-gradient tiles [256 x 256] x 74 splits of every update go through here.
 // blockDim = (32, 8): 128 consecutive output elements per block, the S partials strided over threadIdx.y in the SAME fixed order as
 // reduce_partials_kernel (bit-identical results).  Blocks beyond the matrix reduce the fused column-sum partials (scalar path).
-__global__ void __launch_bounds__(256) reduce_partials_vec4_kernel(const float* __restrict__ partial, int S, int prow, int pcol, int rows, int cols,
-                                                                   float* __restrict__ out, int ld_out, int main_blocks,
-                                                                   const float* __restrict__ vec_partial, float* __restrict__ vec_out,
-                                                                   const float* __restrict__ scale_a, const float* __restrict__ scale_b) {
-    pdl_enter();
+// (the body of one block, `block` = its index in the job's grid: also the per-job blocks of reduce_partials_vec4_multi_kernel)
+__device__ __forceinline__ void reduce_partials_vec4_block(int block, const float* __restrict__ partial, int S, int prow, int pcol, int rows, int cols,
+                                                           float* __restrict__ out, int ld_out, int main_blocks, const float* __restrict__ vec_partial,
+                                                           float* __restrict__ vec_out, const float* __restrict__ scale_a, const float* __restrict__ scale_b) {
     __shared__ float4 red[8][33];
-    if ((int)blockIdx.x >= main_blocks) {  // column-sum tail: one element per thread, as the scalar kernel
+    if (block >= main_blocks) {  // column-sum tail: one element per thread, as the scalar kernel
         const float mul = 1.0f / ld_scale(scale_a);
-        const int e = ((int)blockIdx.x - main_blocks) * 32 + threadIdx.x;
+        const int e = (block - main_blocks) * 32 + threadIdx.x;
         float acc = 0.f;
         if (e < rows) {
             const float* p = vec_partial + e;
@@ -1081,7 +1292,7 @@ __global__ void __launch_bounds__(256) reduce_partials_vec4_kernel(const float* 
         return;
     }
     const float mul = 1.0f / (ld_scale(scale_a) * ld_scale(scale_b));
-    const int e4 = ((int)blockIdx.x * 32 + threadIdx.x) * 4;  // first of this thread's four output elements (row-major over rows x cols)
+    const int e4 = (block * 32 + threadIdx.x) * 4;  // first of this thread's four output elements (row-major over rows x cols)
     const int total = rows * cols;
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     int r = 0, c = 0;
@@ -1134,6 +1345,24 @@ __global__ void __launch_bounds__(256) reduce_partials_vec4_kernel(const float* 
         }
         *reinterpret_cast<float4*>(out + (size_t)r * ld_out + c) = make_float4(t.x * mul, t.y * mul, t.z * mul, t.w * mul);
     }
+}
+
+__global__ void __launch_bounds__(256) reduce_partials_vec4_kernel(const float* __restrict__ partial, int S, int prow, int pcol, int rows, int cols,
+                                                                   float* __restrict__ out, int ld_out, int main_blocks,
+                                                                   const float* __restrict__ vec_partial, float* __restrict__ vec_out,
+                                                                   const float* __restrict__ scale_a, const float* __restrict__ scale_b) {
+    pdl_enter();
+    reduce_partials_vec4_block((int)blockIdx.x, partial, S, prow, pcol, rows, cols, out, ld_out, main_blocks, vec_partial, vec_out, scale_a, scale_b);
+}
+
+// the reductions of every job of a gemm_planes_mn_multi_kernel launch in one grid: job j owns blocks [red_block0, next job's red_block0)
+__global__ void __launch_bounds__(256) reduce_partials_vec4_multi_kernel(const __grid_constant__ MnMulti mj) {
+    pdl_enter();
+    int j = 0;
+    while (j + 1 < mj.n_jobs && (int)blockIdx.x >= mj.job[j + 1].red_block0) ++j;
+    const MnJobArgs& jb = mj.job[j];
+    reduce_partials_vec4_block((int)blockIdx.x - jb.red_block0, jb.partial, jb.S, jb.g_cols, jb.NB, jb.g_cols, jb.h_cols, jb.out, jb.ld_out, jb.red_main_blocks,
+                               jb.colsum_partial, jb.colsum_out, jb.g_scale, jb.h_scale);
 }
 
 // column sums of a plane tensor: part[chunk][n] = sum over the chunk's rows and the P planes of G[p][m][n] (still scaled).
@@ -1573,6 +1802,22 @@ static int make_plane_map_mn(CUtensorMap* map, int fmt, const void* base, int ro
 
 static inline bool fmt_ok(int fmt) { return fmt == MORL_FMT_BF16X3 || fmt == MORL_FMT_F16X2; }
 
+// split-K plan of an MN-major product: S splits of rps rows (a multiple of kMnKT) so that n_tiles * S fills the 148 SMs; no split is empty
+static inline void mn_split(int M, int n_tiles, int& S, int& rps) {
+    S = 148 / n_tiles;
+    if (S < 1) S = 1;
+    rps = ((M + S - 1) / S + kMnKT - 1) / kMnKT * kMnKT;
+    S = (M + rps - 1) / rps;
+}
+
+// floats of a multi-job workspace region: partials [S][g_cols][NB], then the column-sum partials [S][g_cols] (rounded up to 16 bytes)
+static inline size_t mn_multi_job_floats(int M, int g_cols, int h_cols) {
+    int S, rps;
+    mn_split(M, (g_cols + 127) / 128, S, rps);
+    const size_t nb = (size_t)((h_cols + 63) / 64 * 64);
+    return (size_t)S * g_cols * nb + ((size_t)S * g_cols + 3) / 4 * 4;
+}
+
 }  // namespace morl
 
 extern "C" int morl_plane_overflow_count(int reset) {
@@ -1605,10 +1850,8 @@ extern "C" int morl_amax_scale_f32(const float* src, long long n, int target_exp
 extern "C" size_t morl_gemm_mn_workspace_bytes(int M, int a_cols, int b_cols) {
     if (M <= 0 || a_cols <= 0 || b_cols <= 0) return 0;
     const int n_tiles = (a_cols + 127) / 128;
-    int S = 148 / n_tiles;
-    if (S < 1) S = 1;
-    int rps = ((M + S - 1) / S + 31) / 32 * 32;
-    S = (M + rps - 1) / rps;
+    int S, rps;
+    morl::mn_split(M, n_tiles, S, rps);
     const int NB = (b_cols + 63) / 64 * 64;
     return (size_t)S * n_tiles * 128 * NB * sizeof(float) + (size_t)256 * 256 * sizeof(float);  // tail: [S][n_tiles*128] column-sum partials
 }
@@ -1624,10 +1867,8 @@ extern "C" int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long 
                  "morl_gemm_planes_mn_f32: plane row lengths must be multiples of 64 (ldg=%d ldh=%d), ldh <= 256", ldg, ldh);
     const int n_tiles = (g_cols + 127) / 128;
     MORL_REQUIRE(n_tiles * 128 <= ldg || ldg % 128 == 0 || n_tiles * 128 - ldg <= 64, MORL_ERR_UNSUPPORTED, "morl_gemm_planes_mn_f32: ldg=%d", ldg);
-    int S = 148 / n_tiles;
-    if (S < 1) S = 1;
-    const int rps = ((M + S - 1) / S + 31) / 32 * 32;
-    S = (M + rps - 1) / rps;
+    int S, rps;
+    mn_split(M, n_tiles, S, rps);
     const int NB = (h_cols + 63) / 64 * 64;
     CUtensorMap tmA, tmB;
     int rc = make_plane_map_mn(&tmA, fmt, g_planes, M, ldg, g_plane_stride);
@@ -1639,8 +1880,7 @@ extern "C" int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long 
     g.colsum_partial = colsum_out ? g.partial + (size_t)S * n_tiles * 128 * NB : nullptr;  // S * n_tiles * 128 <= 148 * 128 floats < 256 KB tail
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MORL_DISPATCH_FMT(fmt, {
-        using F = PlaneFmt<kFmt>;
-        const size_t smem = (size_t)F::kStagesMn * (6u * F::P * kMnKT * 128u) + 256 + 1024 + 64 + 1024 + 4096;
+        const size_t smem = mn_smem_bytes<kFmt>();
         static bool attr_set = false, attr_set_mc = false;
         if (!attr_set) {
             cudaFuncSetAttribute(gemm_planes_mn_kernel<kFmt, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1687,6 +1927,81 @@ extern "C" int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long 
     launch_k(reduce_partials_kernel, dim3(main_blocks + vec_blocks), dim3(dim3(32, 8)), 0, st, g.partial, S, n_tiles * 128, NB, g_cols, h_cols, transpose_out, out, ld_out,
                                                                              main_blocks, g.colsum_partial, colsum_out, g_scale, h_scale);
     return check_launch("morl_gemm_planes_mn_f32(reduce)");
+}
+
+extern "C" size_t morl_gemm_mn_multi_workspace_bytes(const MorlMnJob* jobs, int n_jobs, int M) {
+    using namespace morl;
+    if (!jobs || n_jobs <= 0 || n_jobs > kMnMaxJobs || M <= 0) return 0;
+    size_t floats = 0;
+    for (int i = 0; i < n_jobs; ++i) {
+        if (jobs[i].g_cols <= 0 || jobs[i].h_cols <= 0) return 0;
+        floats += mn_multi_job_floats(M, jobs[i].g_cols, jobs[i].h_cols);
+    }
+    return floats * sizeof(float);
+}
+
+extern "C" int morl_gemm_planes_mn_multi_f32(int fmt, const MorlMnJob* jobs, int n_jobs, int M, void* workspace, void* stream) {
+    using namespace morl;
+    MORL_REQUIRE(fmt_ok(fmt), MORL_ERR_UNSUPPORTED, "morl_gemm_planes_mn_multi_f32: unknown plane format %d", fmt);
+    MORL_REQUIRE(jobs && workspace, MORL_ERR_NULL, "morl_gemm_planes_mn_multi_f32: NULL pointer argument");
+    MORL_REQUIRE(n_jobs >= 1 && n_jobs <= kMnMaxJobs && M > 0, MORL_ERR_SHAPE, "morl_gemm_planes_mn_multi_f32: bad n_jobs=%d / M=%d (1 <= n_jobs <= %d)", n_jobs, M,
+                 kMnMaxJobs);
+    MORL_REQUIRE(aligned16(workspace), MORL_ERR_ALIGN, "morl_gemm_planes_mn_multi_f32: workspace must be 16-byte aligned");
+    MnMulti mj;  // (host staging; copied into the kernel parameters by the launches)
+    memset(&mj, 0, sizeof(mj));
+    mj.n_jobs = n_jobs;
+    mj.M = M;
+    float* ws = static_cast<float*>(workspace);
+    int units = 0, red_blocks = 0;
+    for (int i = 0; i < n_jobs; ++i) {
+        const MorlMnJob& q = jobs[i];
+        MORL_REQUIRE(q.g_planes && q.h_planes && q.out, MORL_ERR_NULL, "morl_gemm_planes_mn_multi_f32: job %d has a NULL pointer", i);
+        MORL_REQUIRE(q.g_cols > 0 && q.h_cols > 0 && q.ldg % 64 == 0 && q.ldh % 64 == 0 && q.ldh <= 256 && q.g_cols <= q.ldg && q.h_cols <= q.ldh,
+                     MORL_ERR_SHAPE, "morl_gemm_planes_mn_multi_f32: job %d: bad shape g_cols=%d ldg=%d h_cols=%d ldh=%d (ld multiples of 64, ldh <= 256)", i,
+                     q.g_cols, q.ldg, q.h_cols, q.ldh);
+        const int n_tiles = (q.g_cols + 127) / 128;
+        MORL_REQUIRE(n_tiles * 128 <= q.ldg || q.ldg % 128 == 0 || n_tiles * 128 - q.ldg <= 64, MORL_ERR_UNSUPPORTED,
+                     "morl_gemm_planes_mn_multi_f32: job %d: ldg=%d", i, q.ldg);
+        // the reduction stores four consecutive columns per thread
+        MORL_REQUIRE(q.h_cols % 4 == 0 && q.ld_out >= q.h_cols && q.ld_out % 4 == 0 && aligned16(q.out), MORL_ERR_UNSUPPORTED,
+                     "morl_gemm_planes_mn_multi_f32: job %d: needs h_cols %% 4 == 0, ld_out %% 4 == 0 (>= h_cols) and a 16-byte aligned output", i);
+        MnJobArgs& a = mj.job[i];
+        mn_split(M, n_tiles, a.S, a.rows_per_split);
+        a.n_tiles = n_tiles;
+        a.NB = (q.h_cols + 63) / 64 * 64;
+        a.g_cols = q.g_cols; a.h_cols = q.h_cols; a.ld_out = q.ld_out;
+        a.unit0 = units;
+        units += n_tiles * a.S;
+        a.partial = ws;
+        a.colsum_partial = q.colsum_out ? ws + (size_t)a.S * q.g_cols * a.NB : nullptr;
+        ws += mn_multi_job_floats(M, q.g_cols, q.h_cols);
+        a.out = q.out; a.colsum_out = q.colsum_out; a.g_scale = q.g_scale; a.h_scale = q.h_scale;
+        a.red_block0 = red_blocks;
+        a.red_main_blocks = (q.g_cols * q.h_cols / 4 + 31) / 32;
+        red_blocks += a.red_main_blocks + (q.colsum_out ? (q.g_cols + 31) / 32 : 0);
+        int rc = make_plane_map_mn(&mj.tmA[i], fmt, q.g_planes, M, q.ldg, q.g_plane_stride);
+        MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_multi_f32: job %d: cuTensorMapEncodeTiled(G) failed (%d)", i, rc);
+        rc = make_plane_map_mn(&mj.tmB[i], fmt, q.h_planes, M, q.ldh, q.h_plane_stride);
+        MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_multi_f32: job %d: cuTensorMapEncodeTiled(H) failed (%d)", i, rc);
+    }
+    mj.n_units = units;
+    int sms = morl_device_sm_count();
+    if (sms <= 0) sms = 148;
+    const int grid = units < sms ? units : sms;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MORL_DISPATCH_FMT(fmt, {
+        constexpr size_t smem = mn_smem_bytes<kFmt>();
+        static bool attr_set = false;
+        if (!attr_set) {
+            cudaFuncSetAttribute(gemm_planes_mn_multi_kernel<kFmt>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            attr_set = true;
+        }
+        launch_k(gemm_planes_mn_multi_kernel<kFmt>, dim3(grid), dim3(kGemmThreads), smem, st, mj);
+    });
+    const int rc = check_launch("morl_gemm_planes_mn_multi_f32");
+    if (rc) return rc;
+    launch_k(reduce_partials_vec4_multi_kernel, dim3(red_blocks), dim3(32, 8), 0, st, mj);
+    return check_launch("morl_gemm_planes_mn_multi_f32(reduce)");
 }
 
 extern "C" int morl_colsum_planes(int fmt, const void* planes, long long plane_stride, const float* scale, int M, int ld, int N, float* out,

@@ -136,6 +136,12 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
           "=r"(v[31])
         : "r"(taddr));
 }
+// one column of a warp's 32 TMEM lanes (waits for the load)
+__device__ __forceinline__ uint32_t tc_ld1(uint32_t taddr) {
+    uint32_t v;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\n\ttcgen05.wait::ld.sync.aligned;" : "=r"(v) : "r"(taddr) : "memory");
+    return v;
+}
 __device__ __forceinline__ void tc_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // ---- operand formats ------------------------------------------------------------------------------------------------------

@@ -675,6 +675,40 @@ def gemm_planes_mn(g_planes: th.Tensor, g_cols: int, h_planes: th.Tensor, h_cols
     return out
 
 
+class GemmMnMulti:
+    """Static plan of several weight-gradient products over the same rows in ONE persistent launch plus one reduction
+    (morl_gemm_planes_mn_multi_f32): each entry of ``jobs`` is ``(g_planes, g_cols, h_planes, h_cols, out, colsum, g_scale, h_scale)``
+    with the meaning of :func:`gemm_planes_mn` (``colsum`` and the scales may be None; ``out`` is [g_cols, h_cols], not transposed).  Every
+    output is bit-identical to the per-product :func:`gemm_planes_mn` call.  The job table and the workspace are built once; a call is two launches."""
+
+    def __init__(self, jobs):
+        if not 1 <= len(jobs) <= _lib.MN_MAX_JOBS:
+            raise _lib.MorlB200Error(f"GemmMnMulti: 1 to {_lib.MN_MAX_JOBS} products per launch (got {len(jobs)})")
+        self.fmt = fmt_of(jobs[0][0])
+        self.M = jobs[0][0].shape[1]
+        arr = (_lib.MnJob * len(jobs))()
+        for i, (g, gc, h, hc, out, colsum, sg, sh) in enumerate(jobs):
+            if fmt_of(g) != self.fmt or fmt_of(h) != self.fmt or g.shape[1] != self.M or h.shape[1] != self.M:
+                raise _lib.MorlB200Error("GemmMnMulti: plane tensors must share format and number of rows")
+            if tuple(out.shape) != (gc, hc) or out.stride(1) != 1 or out.dtype != th.float32:
+                raise _lib.MorlB200Error(f"GemmMnMulti: job {i}: out must be fp32 [{gc}, {hc}] with unit column stride")
+            if colsum is not None and (colsum.numel() < gc or colsum.dtype != th.float32 or not colsum.is_contiguous()):
+                raise _lib.MorlB200Error(f"GemmMnMulti: job {i}: colsum must be a contiguous fp32 tensor of {gc} elements")
+            arr[i] = _lib.MnJob(_ptr(g), g.stride(0), _ptr(sg), _ptr(h), h.stride(0), _ptr(sh), _ptr(out), _ptr(colsum), g.shape[2], int(gc), h.shape[2],
+                                int(hc), out.stride(0))
+        self._jobs, self._n = arr, len(jobs)
+        self._keep = jobs
+        nbytes = _lib.load().morl_gemm_mn_multi_workspace_bytes(arr, self._n, self.M)
+        if nbytes == 0:
+            raise _lib.MorlB200Error("GemmMnMulti: bad job shapes")
+        self.workspace = th.empty((nbytes + 3) // 4, device=jobs[0][0].device, dtype=th.float32)
+
+    def __call__(self):
+        rc = _lib.load().morl_gemm_planes_mn_multi_f32(self.fmt, self._jobs, self._n, self.M, _ptr(self.workspace), _stream())
+        _lib.check(rc, "morl_gemm_planes_mn_multi_f32")
+        _count(2)
+
+
 def colsum_planes(planes: th.Tensor, n_cols: int, out: Optional[th.Tensor] = None, workspace: Optional[th.Tensor] = None,
                   scale: Optional[th.Tensor] = None) -> th.Tensor:
     """Column sums over the rows and the planes, scale removed (bias gradients)."""

@@ -47,6 +47,7 @@ from . import ops
 _SNAKE = os.environ.get("MORL_TC_SNAKE", "1") == "1"          # alternate the GEMM tile order between chained layers
 _CHAIN = os.environ.get("MORL_GEMM_CHAIN", "1") == "1"        # hidden layers 2.. of a pass as ONE chained launch (+10 % on the update; =0: one launch per layer)
 _CHAIN_BWD = os.environ.get("MORL_GEMM_CHAIN_BWD", "1") == "1"  # ... and the 256-wide dX products of the backward pass (+2.7 %; =0: per-layer launches)
+_MN_MULTI = os.environ.get("MORL_MN_MULTI", "1") == "1"          # ... and all weight-gradient products of it as ONE launch + one reduction (=0: per layer)
 _NARROW_HEAD = os.environ.get("MORL_NARROW_HEAD", "1") == "1"  # output layer through morl_qhead_gemm_f32 (19.7 us against 26 us in the update; =0: general kernel)
 _DEFAULT_FMT = ops.FMT_BF16X3 if os.environ.get("MORL_TC_FMT", "f16x2") == "bf16x3" else ops.FMT_F16X2
 
@@ -108,7 +109,7 @@ class TCPairMlp:
             self.wp = [ops.empty_planes(fmt, _pad(l.out_features, 32), l.in_features, dev) for l in self.lin[1:]]
             self.s_w = [ops.scale_tensor(1.0, dev) if scaled else None for _ in self.lin[1:]]
         self.q = th.empty((M, self.lin[-1].out_features), device=dev, dtype=th.float32)
-        self._chain = self._gchain = self._gbufs = None
+        self._chain = self._gchain = self._gbufs = self._mn_multi = None
         self.trainable = trainable
         if trainable:
             if n_w > 64:
@@ -287,7 +288,8 @@ class TCPairMlp:
 def _backward_chained(self, feats, wset, G, grads, after_gemms):
     """Backward with the 256-wide dX products as ONE chained launch: G_{n-2} from the (narrow) output layer as before, then
     G_{k-1} = (G_k . W_k) * relu'(H_{k-1}) for k = n-2 .. 1 in one persistent kernel (each G_k in its own buffer: the weight-gradient
-    products read them afterwards), then the n-1 weight-gradient GEMMs."""
+    products read them afterwards), then the n-1 weight-gradient GEMMs -- one multi-job launch (ops.GemmMnMulti), or per layer with
+    MORL_MN_MULTI=0 (the output layer's before the chain)."""
     n = len(self.lin)
     dev = G.device
     if self._gchain is None:
@@ -297,26 +299,46 @@ def _backward_chained(self, feats, wset, G, grads, after_gemms):
         ks = list(range(n - 1, 0, -1))  # layers whose dX product is in the chain: the narrow output layer first
         self._gchain = ops.GemmChain([[self.g_last] + self._gbufs], [[self.wtp[k - 1] for k in ks]], None, [[self.s_w[k - 1] for k in ks]], None,
                                      act_scale=self.s_g, relu=False, bits_in=[[self.hbits[k - 1] for k in ks]], k_first=self.ld_last)
+    for k in range(1, n):
+        if grads[2 * k] is None:
+            grads[2 * k] = th.empty((self.lin[k].out_features, self.lin[k].in_features), device=dev, dtype=th.float32)
+        if grads[2 * k + 1] is None:
+            grads[2 * k + 1] = th.empty(self.lin[k].out_features, device=dev, dtype=th.float32)
+    if _MN_MULTI and n - 1 <= ops._lib.MN_MAX_JOBS:
+        self._gchain()  # all n - 1 dX products (the narrow one of the output layer included) in one launch
+        key = tuple(grads[i].data_ptr() for i in range(2, 2 * n))
+        if self._mn_multi is None or self._mn_multi[0] != key:
+            # dL/dh_k is _gbufs[n - 2 - k]; the chain writes _gbufs[n - 3] (dW of lin[1]) last, so that product goes first (part of its G may
+            # still be in L2), the narrow output layer last
+            jobs = [(self._gbufs[n - 2 - k], self.lin[k].out_features, self.h[k - 1], self.lin[k].in_features, grads[2 * k], grads[2 * k + 1], self.s_g,
+                     self.s_act) for k in range(1, n - 1)]
+            jobs.append((G, self.lin[n - 1].out_features, self.h[n - 2], self.lin[n - 1].in_features, grads[2 * (n - 1)], grads[2 * (n - 1) + 1], self.s_g,
+                         self.s_act))
+            self._mn_multi = (key, ops.GemmMnMulti(jobs))
+        self._mn_multi[1]()
+        return self._backward_tail(feats, wset, grads, after_gemms)
     last = self.lin[n - 1]
-    if grads[2 * (n - 1) + 1] is None:
-        grads[2 * (n - 1) + 1] = th.empty(last.out_features, device=dev, dtype=th.float32)
     grads[2 * (n - 1)] = ops.gemm_planes_mn(G, last.out_features, self.h[n - 2], last.in_features, out=grads[2 * (n - 1)], workspace=self.ws_mn,
                                             colsum=grads[2 * (n - 1) + 1], g_scale=self.s_g, h_scale=self.s_act)
     self._gchain()  # all n - 1 dX products (the narrow one of the output layer included) in one launch
     for i, k in enumerate(range(n - 2, 0, -1)):  # dW_k = (dL/dh_k)^T H_{k-1}: dL/dh_k is _gbufs[i]
         l = self.lin[k]
-        if grads[2 * k + 1] is None:
-            grads[2 * k + 1] = th.empty(l.out_features, device=dev, dtype=th.float32)
         grads[2 * k] = ops.gemm_planes_mn(self._gbufs[i], l.out_features, self.h[k - 1], l.in_features, out=grads[2 * k], workspace=self.ws_mn,
                                           colsum=grads[2 * k + 1], g_scale=self.s_g, h_scale=self.s_act)
+    return self._backward_tail(feats, wset, grads, after_gemms)
+
+
+def _backward_tail(self, feats, wset, grads, after_gemms):
+    """After the last tensor-core GEMM of the chained backward: fork the side work, then the layer-1 gradients."""
     if after_gemms is not None:
         after_gemms()
-    dU, dV = ops.pairs_grad_reduce(self._gbufs[n - 2], self.B, self.W, workspace=self.ws_red, dU=self.dU, dV=self.dV, scale=self.s_g)
+    dU, dV = ops.pairs_grad_reduce(self._gbufs[len(self.lin) - 2], self.B, self.W, workspace=self.ws_red, dU=self.dU, dV=self.dV, scale=self.s_g)
     grads[0], grads[1] = ops.pair_layer1_grad(dU, dV, feats, wset, dW1=grads[0], db1=grads[1], workspace=self.ws_l1)
     return grads
 
 
 TCPairMlp._backward_chained = _backward_chained
+TCPairMlp._backward_tail = _backward_tail
 
 
 class TCPairMlpFn(th.autograd.Function):

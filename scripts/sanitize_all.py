@@ -2,7 +2,7 @@
 
     compute-sanitizer --tool memcheck|racecheck|synccheck|initcheck python scripts/sanitize_all.py [group ...]
 
-groups: envelope td gemm optim pareto replay layer1 qhead dyna chain (default: all).  Shapes are small (sanitizer slows kernels 10-100x) but exercise
+groups: envelope td gemm optim pareto replay layer1 qhead dyna chain mn_multi (default: all).  Shapes are small (sanitizer slows kernels 10-100x) but exercise
 every code path: all envelope kernel families, both GEMM operand formats x CTA modes x accumulator modes, MN split-K GEMM with the fused
 column sums, every split / reduction helper, the loss kernels, Adam, polyak, Pareto + front records, replay gather."""
 import os
@@ -22,7 +22,7 @@ if os.environ.get("SAN_ZERO_PLANES") == "1":
     # from a genuine read of memory nobody wrote (profiles/r02_sanitize_initcheck*.txt).
     _empty = ops.empty_planes
     ops.empty_planes = lambda *a, **k: _empty(*a, **k).zero_()
-groups = set(sys.argv[1:]) or {"envelope", "td", "gemm", "optim", "pareto", "replay", "layer1", "qhead", "dyna", "chain"}
+groups = set(sys.argv[1:]) or {"envelope", "td", "gemm", "optim", "pareto", "replay", "layer1", "qhead", "dyna", "chain", "mn_multi"}
 
 
 def rn(*s, scale=1.0):
@@ -194,4 +194,23 @@ if "chain" in groups:
     ops.GemmChain([gb], [ws[0]], None, [sws[0]], None, act_scale=sa, relu=False, bits_in=[bits[0]])()
     th.cuda.synchronize()
     print("chain ok")
+if "mn_multi" in groups:
+    # multi-job weight-gradient launch (gemm_planes_mn_multi_kernel + reduce_partials_vec4_multi_kernel): 220 units on at most 148 CTAs, so
+    # CTAs take several units (ring and accumulator phases wrap across units of different jobs); a 24-wide job with trimmed partial rows
+    M = 6000
+    for fmt in (ops.FMT_F16X2, ops.FMT_BF16X3):
+        sg = ops.scale_tensor(2.0**16, dev) if fmt == ops.FMT_F16X2 else None
+        sa = ops.scale_tensor(2.0, dev) if fmt == ops.FMT_F16X2 else None
+        jobs, ref = [], []
+        for gc, hc, ldg, colsum in ((256, 128, 256, True), (24, 128, 64, True), (64, 64, 64, False)):
+            Gp = ops.split_planes(rn(M, gc, scale=1e-3), fmt, ldp=ldg, scale=sg)
+            Hp = ops.split_planes(rn(M, hc).relu_(), fmt, scale=sa)
+            cs = th.empty(gc, device=dev) if colsum else None
+            ref.append((ops.gemm_planes_mn(Gp, gc, Hp, hc, colsum=cs, g_scale=sg, h_scale=sa), cs))
+            jobs.append((Gp, gc, Hp, hc, th.empty(gc, hc, device=dev), th.empty(gc, device=dev) if colsum else None, sg, sa))
+        ops.GemmMnMulti(jobs)()
+        th.cuda.synchronize()
+        for (dW, cs), j in zip(ref, jobs):
+            assert th.equal(j[4], dW) and (cs is None or th.equal(j[5], cs))
+    print("mn_multi ok")
 print("sanitize run ok")
