@@ -381,15 +381,17 @@ MORL_API int morl_pairs_relu_split_planes(int fmt, const float* u, const float* 
  *   scaled by *h_scale);  ldg, ldh multiples of 64, ldh <= 256;  transpose_out != 0 stores out[k, n] instead.  Replaces the
  *   dW = dY^T X products that torch autograd issues for the nn.Linear layers of the reference networks (loss.backward(), envelope.py:316).
  *   colsum_out (nullable, [g_cols]): out_b[n] = sum_m G[m, n], the bias gradient db = colsum(dY), evaluated in the same pass as
- *   G^T . ones on the tensor cores (replaces a separate sweep of the G planes).
- *   workspace: morl_gemm_mn_workspace_bytes(M, g_cols, h_cols) bytes. */
+ *   G^T . ones on the tensor cores (replaces a separate sweep of the G planes).  Runs as a one-job launch of
+ *   morl_gemm_planes_mn_multi_f32's kernel, then one reduction launch.
+ *   workspace: morl_gemm_mn_workspace_bytes(M, g_cols, h_cols) bytes, 16-byte aligned (MORL_ERR_ALIGN otherwise). */
 MORL_API size_t morl_gemm_mn_workspace_bytes(int M, int a_cols, int b_cols);
 MORL_API int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long g_plane_stride, int ldg, int g_cols, const float* g_scale,
                                      const void* h_planes, long long h_plane_stride, int ldh, int h_cols, const float* h_scale, int M,
                                      int transpose_out, float* out, int ld_out, float* colsum_out, void* workspace, void* stream);
 /* Up to MORL_MN_MAX_JOBS weight-gradient products over the same M rows in ONE persistent launch plus ONE reduction launch: job j computes
- * out[n, k] (and colsum_out[n]) exactly as morl_gemm_planes_mn_f32 with transpose_out = 0 does -- bit-identical -- but the operand stream does
- * not stop between the products (the backward pass of an update: the output layer and every hidden layer).  Per job: ldg, ldh multiples of
+ * out[n, k] (and colsum_out[n]) bit-identically to morl_gemm_planes_mn_f32 with transpose_out = 0 on that job alone (the same kernel; a job's
+ * splits and summation order do not depend on the other jobs), but the operand stream does not stop between the products (the backward pass
+ * of an update: the output layer and every hidden layer).  Per job: ldg, ldh multiples of
  * 64, ldh <= 256, h_cols % 4 == 0, ld_out % 4 == 0, out 16-byte aligned (others are refused with MORL_ERR_UNSUPPORTED); colsum_out nullable.
  *   workspace: morl_gemm_mn_multi_workspace_bytes(jobs, n_jobs, M) bytes, 16-byte aligned. */
 #define MORL_MN_MAX_JOBS 4

@@ -816,9 +816,9 @@ gemm_chain_kernel(const __grid_constant__ ChainMaps maps, const ChainArgs g) {
 // =================================================================================================================
 // MN-major split-K variant: weight gradients  dW[n, k] = sum_m G[m, n] * H[m, k]  (reduction over the 65,536 batch rows).
 // Both operands are the row-major plane tensors the forward/backward GEMMs already produced, read "MN-major" (the MMA's M / N
-// index is the contiguous one), 128-byte swizzle:  A = G^T (M_mma = n, 128 per CTA), B = H^T (N_mma = k <= 256), K_mma = m.
-// One CTA per (128-row block of n, split s of the m range); fp32 partial tiles are summed by reduce_partials_kernel
-// (deterministic, no atomics), which also removes the operand scales.
+// index is the contiguous one), 128-byte swizzle:  A = G^T (M_mma = n, 128 per unit), B = H^T (N_mma = k <= 256), K_mma = m.
+// A unit of work is (128-row block of n, split s of the m range); its fp32 partial tile is summed over the splits by a separate
+// reduction launch (deterministic, no atomics), which also removes the operand scales.
 // =================================================================================================================
 constexpr int kMnKT = 32;  // batch rows (K_mma direction) per pipeline stage
 
@@ -834,168 +834,7 @@ __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr, uint3
     return d;
 }
 
-struct GemmMnArgs {
-    int M;            // reduction length (batch rows)
-    int n_tiles;      // ceil(A columns / 128)
-    int NB;           // N_mma = B columns covered (multiple of 64, <= 256)
-    int rows_per_split;
-    float* partial;   // [S][n_tiles*128][NB]
-    float* colsum_partial;  // [S][n_tiles*128] or nullptr: per-split column sums of G (bias gradient), fused as G^T . ones
-};
-
-// MC = 1 (two column tiles, NB = 256): the two CTAs of a split (column tiles 0 and 1: consecutive blocks) form a CLUSTER; each loads its own
-// 128 G columns and HALF of the H chunks, multicast to both CTAs, so H crosses the L2 -> SM path once per split instead of twice.  The kernel
-// (hypothesis: 67 MB of G + 2 x 67 MB of H per launch through that path at ~6.5 TB/s would explain the 31 us measured.  Built, correct, and
-// measured: no gain, see the launcher -- opt-in.)
-// A stage may be refilled only when BOTH CTAs have consumed it: every MMA commit arrives on the stage's empty barrier of both CTAs.
-template <int FMT, int MC>
-__global__ void __launch_bounds__(192, 1)
-gemm_planes_mn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmMnArgs g) {
-    using F = PlaneFmt<FMT>;
-    constexpr int P = F::P;
-    constexpr int kStages = F::kStagesMn;
-    extern __shared__ uint8_t gsmem_raw[];
-    // 1 KB alignment by pointer arithmetic ON the shared array (not through an integer cast), so that the compiler keeps every derived
-    // pointer in the shared address space: through the cast the bias / staging accesses were generic LD.E / ST.E (long-scoreboard stalls)
-    uint8_t* gsmem = gsmem_raw + ((1024u - (g_smem_u32(gsmem_raw) & 1023u)) & 1023u);
-    constexpr uint32_t chunk_bytes = (uint32_t)P * kMnKT * 128u;   // one 64-element MN chunk, P planes
-    constexpr uint32_t a_stage = 2u * chunk_bytes;
-    constexpr uint32_t b_stage = 4u * chunk_bytes;                 // (allocated for NB = 256)
-    const int nb_chunks = g.NB / 64;
-    uint8_t* smA = gsmem;
-    uint8_t* smB = gsmem + kStages * a_stage;
-    uint64_t* full = reinterpret_cast<uint64_t*>(smB + kStages * b_stage);
-    uint64_t* empty = full + kStages;
-    uint64_t* tfull = empty + kStages;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tfull + 1);
-    // 4 KB of 1.0: the B operand of the fused bias-gradient product  colsum(G) = G^T . ones  (N = 16; every element is 1,
-    // so the swizzle pattern is irrelevant)
-    uint8_t* ones_b = reinterpret_cast<uint8_t*>(tmem_slot + 4);
-    uint32_t* ones = reinterpret_cast<uint32_t*>(ones_b + ((1024u - (g_smem_u32(ones_b) & 1023u)) & 1023u));
-    for (int t = threadIdx.x; t < 1024; t += blockDim.x) ones[t] = F::kOnes2;
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int nt = blockIdx.x % g.n_tiles;
-    const int split = blockIdx.x / g.n_tiles;
-    const int m_begin = split * g.rows_per_split;
-    const int m_end = min(g.M, m_begin + g.rows_per_split);
-    const int n_kblk = (m_end - m_begin + kMnKT - 1) / kMnKT;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < kStages; ++s) {
-            g_mbar_init(&full[s], 1);
-            g_mbar_init(&empty[s], MC ? 2 : 1);  // MC: released by the MMA commits of both CTAs of the cluster
-        }
-        g_mbar_init(tfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {  // 256 accumulator columns + 16 for the fused column sums (allocation granularity: power of two)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(g_smem_u32(tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (MC) cluster_sync_all();  // the peer's barriers exist before any multicast copy / remote arrive targets them
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    pdl_enter();  // (nothing above reads or writes global memory: barriers, the tile of ones and the TMEM allocation overlap the predecessor)
-
-    if (warp == 0) {
-        if (lane == 0) {
-            uint32_t stage = 0, phase = 0;
-            for (int kb = 0; kb < n_kblk; ++kb) {
-                g_mbar_wait(&empty[stage], phase ^ 1u);
-                g_mbar_expect_tx(&full[stage], (2u + (uint32_t)nb_chunks) * chunk_bytes);
-                const int m0 = m_begin + kb * kMnKT;
-                for (int c = 0; c < 2; ++c) tma_load_3d(smA + stage * a_stage + c * chunk_bytes, &tmA, &full[stage], nt * 128 + c * 64, m0, 0);
-                if (MC) {
-                    // this CTA fetches H chunks 2 nt, 2 nt + 1 for BOTH CTAs (same shared-memory offset and barrier offset in each); the other
-                    // two chunks arrive from the peer's multicast -- every full barrier still counts 2 + 4 chunks
-                    for (int c = 2 * nt; c < 2 * nt + 2; ++c)
-                        tma_load_3d_multicast(smB + stage * b_stage + c * chunk_bytes, &tmB, &full[stage], c * 64, m0, 0, (uint16_t)3);
-                } else {
-                    for (int c = 0; c < nb_chunks; ++c) tma_load_3d(smB + stage * b_stage + c * chunk_bytes, &tmB, &full[stage], c * 64, m0, 0);
-                }
-                if (++stage == kStages) {
-                    stage = 0;
-                    phase ^= 1u;
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            // D=f32, A/B of the plane type, both MN-major, N = NB, M = 128
-            const uint32_t idesc = (1u << 4) | F::kIdescAB | (1u << 15) | (1u << 16) | ((uint32_t)(g.NB >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-            const uint32_t idesc_ones = (1u << 4) | F::kIdescAB | (1u << 15) | (1u << 16) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-            const uint64_t ones_desc = make_desc_mn_sw128(g_smem_u32(ones), chunk_bytes);
-            constexpr uint32_t plane = kMnKT * 128u;  // 4 KB: one plane of one chunk
-            uint32_t stage = 0, phase = 0;
-            for (int kb = 0; kb < n_kblk; ++kb) {
-                g_mbar_wait(&full[stage], phase);
-                tc_fence_after();
-                const uint32_t a0 = g_smem_u32(smA + stage * a_stage);
-                const uint32_t b0 = g_smem_u32(smB + stage * b_stage);
-#pragma unroll
-                for (int ks = 0; ks < kMnKT / 16; ++ks) {
-#pragma unroll
-                    for (int t = 0; t < F::NPROD; ++t) {
-                        const uint64_t ad = make_desc_mn_sw128(a0 + F::pa(t) * plane + ks * 2048u, chunk_bytes);
-                        const uint64_t bd = make_desc_mn_sw128(b0 + F::pb(t) * plane + ks * 2048u, chunk_bytes);
-                        tc_mma_bf16(tmem_base, ad, bd, idesc, (kb | ks | t) != 0 ? 1u : 0u);
-                    }
-                    if (g.colsum_partial) {  // (G_{P-1} + ... + G_0)^T . ones -> 16 identical columns at TMEM column 256
-#pragma unroll
-                        for (int pl = P - 1; pl >= 0; --pl)
-                            tc_mma_bf16(tmem_base + 256u, make_desc_mn_sw128(a0 + pl * plane + ks * 2048u, chunk_bytes), ones_desc, idesc_ones,
-                                        (kb | ks | (P - 1 - pl)) != 0 ? 1u : 0u);
-                    }
-                }
-                if (MC) tc_commit_mc(&empty[stage]); else tc_commit(&empty[stage]);
-                if (++stage == kStages) {
-                    stage = 0;
-                    phase ^= 1u;
-                }
-            }
-            tc_commit(tfull);
-        }
-    } else {
-        const int quad = warp & 3;
-        g_mbar_wait(tfull, 0);
-        tc_fence_after();
-        const int row = nt * 128 + quad * 32 + lane;  // output row (n)
-        float* prow = g.partial + ((size_t)split * g.n_tiles * 128 + row) * g.NB;
-        const uint32_t t_row = tmem_base + ((uint32_t)(quad * 32) << 16);
-        for (int n0 = 0; n0 < g.NB; n0 += 32) {
-            uint32_t v[32];
-            tc_ld32(t_row + (uint32_t)n0, v);
-            tc_ld_wait();
-            if (n_kblk > 0) {
-#pragma unroll
-                for (int j = 0; j < 32; j += 4)
-                    *reinterpret_cast<float4*>(prow + n0 + j) = make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
-            } else {
-#pragma unroll
-                for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(prow + n0 + j) = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-        }
-        if (g.colsum_partial) {
-            uint32_t v[32];
-            tc_ld32(t_row + 256u, v);
-            tc_ld_wait();
-            g.colsum_partial[(size_t)split * g.n_tiles * 128 + row] = n_kblk > 0 ? __uint_as_float(v[0]) : 0.f;
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (MC) cluster_sync_all();  // no CTA exits while its peer may still multicast into it or arrive on its barriers
-    if (warp == 1) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
-    }
-}
-
-// shared memory of the MN-major kernels: the TMA ring (A: 2 chunks, B: up to 4 chunks per stage), barriers, the 4 KB tile of ones, slack
+// shared memory of the MN-major kernel: the TMA ring (A: 2 chunks, B: up to 4 chunks per stage), barriers, the 4 KB tile of ones, slack
 template <int FMT>
 constexpr size_t mn_smem_bytes() {
     return (size_t)PlaneFmt<FMT>::kStagesMn * (6u * PlaneFmt<FMT>::P * kMnKT * 128u) + 256 + 1024 + 64 + 1024 + 4096;
@@ -1003,10 +842,11 @@ constexpr size_t mn_smem_bytes() {
 
 // -----------------------------------------------------------------------------------------------------------------
 // Several weight-gradient products  dW_j = G_j^T H_j (+ db_j = colsum(G_j))  in ONE persistent launch (the backward pass of an update:
-// the output layer and every hidden layer).  A unit is (job, column tile, split) with exactly the split boundaries, MMA shape and MMA issue
-// order of gemm_planes_mn_kernel, so every partial is bit-identical to the per-layer launch; units are dealt round-robin to the CTAs.  What
-// the launch gains is continuity: the TMA ring streams the next unit's operands while the current unit's MMAs and epilogue run, and the
-// prologue (barriers, TMEM allocation, tile of ones) is paid once instead of once per layer.
+// the output layer and every hidden layer), or one product alone (morl_gemm_planes_mn_f32).  A unit is (job, column tile, split); a job's
+// split boundaries, MMA shape and MMA issue order do not depend on the other jobs of the launch, so every partial is the same whether the
+// product runs alone or with others; units are dealt round-robin to the CTAs.  What a launch of several jobs gains is continuity: the TMA
+// ring streams the next unit's operands while the current unit's MMAs and epilogue run, and the prologue (barriers, TMEM allocation, tile
+// of ones) is paid once instead of once per layer.
 // The accumulator (256 + 16 columns) cannot be double-buffered in 512 TMEM columns: the 8 epilogue warps copy it to registers (two warps per
 // lane quadrant, half of the columns each), release it, and store the partials while the MMAs of the next unit already run.
 // Only the real rows (n < g_cols) of a tile are stored: partials are [S][g_cols][NB].
@@ -1014,7 +854,7 @@ constexpr size_t mn_smem_bytes() {
 constexpr int kMnMaxJobs = MORL_MN_MAX_JOBS;
 
 struct MnJobArgs {
-    int n_tiles, NB, rows_per_split, S;  // as GemmMnArgs
+    int n_tiles, NB, rows_per_split, S;  // column tiles of 128, N_mma (h_cols rounded up to 64), batch rows per split, splits
     int g_cols, h_cols, ld_out;
     int unit0;                           // first unit of the job in the launch's unit sequence
     int red_block0, red_main_blocks;     // reduction launch: first block of the job; blocks of the matrix part (column-sum blocks follow)
@@ -1060,7 +900,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_planes_mn_multi_kernel(c
         while (j + 1 < mj.n_jobs && u >= mj.job[j + 1].unit0) ++j;
         return j;
     };
-    // unit u -> job j, column tile nt, split (numbered like the blocks of gemm_planes_mn_kernel) and its row range
+    // unit u -> job j, column tile nt, split and its row range
     auto unit_of = [&](int u, int& j, int& nt, int& split, int& m_begin, int& n_kblk) {
         j = job_of(u);
         const MnJobArgs& jb = mj.job[j];
@@ -1261,7 +1101,7 @@ __global__ void __launch_bounds__(256) reduce_partials_kernel(const float* __res
 // for the non-transposed case with cols % 4 == 0 -- the weight-gradient tiles [256 x 256] x 74 splits of every update go through here.
 // blockDim = (32, 8): 128 consecutive output elements per block, the S partials strided over threadIdx.y in the SAME fixed order as
 // reduce_partials_kernel (bit-identical results).  Blocks beyond the matrix reduce the fused column-sum partials (scalar path).
-// (the body of one block, `block` = its index in the job's grid: also the per-job blocks of reduce_partials_vec4_multi_kernel)
+// (the body of one block of reduce_partials_vec4_multi_kernel, `block` = its index among the blocks of its job)
 __device__ __forceinline__ void reduce_partials_vec4_block(int block, const float* __restrict__ partial, int S, int prow, int pcol, int rows, int cols,
                                                            float* __restrict__ out, int ld_out, int main_blocks, const float* __restrict__ vec_partial,
                                                            float* __restrict__ vec_out, const float* __restrict__ scale_a, const float* __restrict__ scale_b) {
@@ -1345,14 +1185,6 @@ __device__ __forceinline__ void reduce_partials_vec4_block(int block, const floa
         }
         *reinterpret_cast<float4*>(out + (size_t)r * ld_out + c) = make_float4(t.x * mul, t.y * mul, t.z * mul, t.w * mul);
     }
-}
-
-__global__ void __launch_bounds__(256) reduce_partials_vec4_kernel(const float* __restrict__ partial, int S, int prow, int pcol, int rows, int cols,
-                                                                   float* __restrict__ out, int ld_out, int main_blocks,
-                                                                   const float* __restrict__ vec_partial, float* __restrict__ vec_out,
-                                                                   const float* __restrict__ scale_a, const float* __restrict__ scale_b) {
-    pdl_enter();
-    reduce_partials_vec4_block((int)blockIdx.x, partial, S, prow, pcol, rows, cols, out, ld_out, main_blocks, vec_partial, vec_out, scale_a, scale_b);
 }
 
 // the reductions of every job of a gemm_planes_mn_multi_kernel launch in one grid: job j owns blocks [red_block0, next job's red_block0)
@@ -1810,12 +1642,61 @@ static inline void mn_split(int M, int n_tiles, int& S, int& rps) {
     S = (M + rps - 1) / rps;
 }
 
-// floats of a multi-job workspace region: partials [S][g_cols][NB], then the column-sum partials [S][g_cols] (rounded up to 16 bytes)
+// floats of one job's workspace region: partials [S][g_cols][NB], then the column-sum partials [S][g_cols] (rounded up to 16 bytes)
 static inline size_t mn_multi_job_floats(int M, int g_cols, int h_cols) {
     int S, rps;
     mn_split(M, (g_cols + 127) / 128, S, rps);
     const size_t nb = (size_t)((h_cols + 63) / 64 * 64);
     return (size_t)S * g_cols * nb + ((size_t)S * g_cols + 3) / 4 * 4;
+}
+
+// Checks job q as job mj.n_jobs of a launch (messages name the entry point `fn`) and appends it: its MnJobArgs and tensor maps, its partials
+// at `ws`, its reduction blocks after the first `red_blocks` of the launch.  `ws` and `red_blocks` advance past the job.
+static int mn_add_job(const char* fn, int fmt, const MorlMnJob& q, MnMulti& mj, float*& ws, int& red_blocks) {
+    const int i = mj.n_jobs, M = mj.M;
+    MORL_REQUIRE(q.g_planes && q.h_planes && q.out, MORL_ERR_NULL, "%s: job %d has a NULL pointer", fn, i);
+    MORL_REQUIRE(q.g_cols > 0 && q.h_cols > 0 && q.ldg % 64 == 0 && q.ldh % 64 == 0 && q.ldh <= 256 && q.g_cols <= q.ldg && q.h_cols <= q.ldh,
+                 MORL_ERR_SHAPE, "%s: job %d: bad shape g_cols=%d ldg=%d h_cols=%d ldh=%d (ld multiples of 64, ldh <= 256)", fn, i, q.g_cols, q.ldg,
+                 q.h_cols, q.ldh);
+    const int n_tiles = (q.g_cols + 127) / 128;
+    MORL_REQUIRE(n_tiles * 128 <= q.ldg || q.ldg % 128 == 0 || n_tiles * 128 - q.ldg <= 64, MORL_ERR_UNSUPPORTED, "%s: job %d: ldg=%d", fn, i, q.ldg);
+    MnJobArgs& a = mj.job[i];
+    mn_split(M, n_tiles, a.S, a.rows_per_split);  // no split is empty: every unit writes its whole partial tile (the reduction reads all S)
+    a.n_tiles = n_tiles;
+    a.NB = (q.h_cols + 63) / 64 * 64;
+    a.g_cols = q.g_cols; a.h_cols = q.h_cols; a.ld_out = q.ld_out;
+    a.unit0 = mj.n_units;
+    mj.n_units += n_tiles * a.S;
+    a.partial = ws;
+    a.colsum_partial = q.colsum_out ? ws + (size_t)a.S * q.g_cols * a.NB : nullptr;
+    ws += mn_multi_job_floats(M, q.g_cols, q.h_cols);
+    a.out = q.out; a.colsum_out = q.colsum_out; a.g_scale = q.g_scale; a.h_scale = q.h_scale;
+    a.red_block0 = red_blocks;
+    a.red_main_blocks = (q.g_cols * q.h_cols / 4 + 31) / 32;
+    red_blocks += a.red_main_blocks + (q.colsum_out ? (q.g_cols + 31) / 32 : 0);
+    int rc = make_plane_map_mn(&mj.tmA[i], fmt, q.g_planes, M, q.ldg, q.g_plane_stride);
+    MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "%s: job %d: cuTensorMapEncodeTiled(G) failed (%d)", fn, i, rc);
+    rc = make_plane_map_mn(&mj.tmB[i], fmt, q.h_planes, M, q.ldh, q.h_plane_stride);
+    MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "%s: job %d: cuTensorMapEncodeTiled(H) failed (%d)", fn, i, rc);
+    mj.n_jobs = i + 1;
+    return 0;
+}
+
+// gemm_planes_mn_multi_kernel over every unit of mj: one CTA per SM, or one per unit when there are fewer units
+static int mn_launch(const char* fn, int fmt, const MnMulti& mj, cudaStream_t st) {
+    int sms = morl_device_sm_count();
+    if (sms <= 0) sms = 148;
+    const int grid = mj.n_units < sms ? mj.n_units : sms;
+    MORL_DISPATCH_FMT(fmt, {
+        constexpr size_t smem = mn_smem_bytes<kFmt>();
+        static bool attr_set = false;
+        if (!attr_set) {
+            cudaFuncSetAttribute(gemm_planes_mn_multi_kernel<kFmt>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            attr_set = true;
+        }
+        launch_k(gemm_planes_mn_multi_kernel<kFmt>, dim3(grid), dim3(kGemmThreads), smem, st, mj);
+    });
+    return check_launch(fn);
 }
 
 }  // namespace morl
@@ -1849,11 +1730,7 @@ extern "C" int morl_amax_scale_f32(const float* src, long long n, int target_exp
 
 extern "C" size_t morl_gemm_mn_workspace_bytes(int M, int a_cols, int b_cols) {
     if (M <= 0 || a_cols <= 0 || b_cols <= 0) return 0;
-    const int n_tiles = (a_cols + 127) / 128;
-    int S, rps;
-    morl::mn_split(M, n_tiles, S, rps);
-    const int NB = (b_cols + 63) / 64 * 64;
-    return (size_t)S * n_tiles * 128 * NB * sizeof(float) + (size_t)256 * 256 * sizeof(float);  // tail: [S][n_tiles*128] column-sum partials
+    return morl::mn_multi_job_floats(M, a_cols, b_cols) * sizeof(float);
 }
 
 extern "C" int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long g_plane_stride, int ldg, int g_cols, const float* g_scale,
@@ -1867,65 +1744,27 @@ extern "C" int morl_gemm_planes_mn_f32(int fmt, const void* g_planes, long long 
                  "morl_gemm_planes_mn_f32: plane row lengths must be multiples of 64 (ldg=%d ldh=%d), ldh <= 256", ldg, ldh);
     const int n_tiles = (g_cols + 127) / 128;
     MORL_REQUIRE(n_tiles * 128 <= ldg || ldg % 128 == 0 || n_tiles * 128 - ldg <= 64, MORL_ERR_UNSUPPORTED, "morl_gemm_planes_mn_f32: ldg=%d", ldg);
-    int S, rps;
-    mn_split(M, n_tiles, S, rps);
-    const int NB = (h_cols + 63) / 64 * 64;
-    CUtensorMap tmA, tmB;
-    int rc = make_plane_map_mn(&tmA, fmt, g_planes, M, ldg, g_plane_stride);
-    MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_f32: cuTensorMapEncodeTiled(G) failed (%d)", rc);
-    rc = make_plane_map_mn(&tmB, fmt, h_planes, M, ldh, h_plane_stride);
-    MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_f32: cuTensorMapEncodeTiled(H) failed (%d)", rc);
-    GemmMnArgs g;
-    g.M = M; g.n_tiles = n_tiles; g.NB = NB; g.rows_per_split = rps; g.partial = static_cast<float*>(workspace);
-    g.colsum_partial = colsum_out ? g.partial + (size_t)S * n_tiles * 128 * NB : nullptr;  // S * n_tiles * 128 <= 148 * 128 floats < 256 KB tail
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MORL_DISPATCH_FMT(fmt, {
-        const size_t smem = mn_smem_bytes<kFmt>();
-        static bool attr_set = false, attr_set_mc = false;
-        if (!attr_set) {
-            cudaFuncSetAttribute(gemm_planes_mn_kernel<kFmt, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            attr_set = true;
-        }
-        // measured (profiles/r02_bench_ab_mn_multicast.txt): correct, but the update does not get faster (1,558 vs 1,558 / 1,564 updates/s) -- the
-        // kernel is not bound by the L2 -> SM path of H after all -> opt-in (MORL_MN_MULTICAST=1), the single-CTA form stays the default
-        static const bool mc_env = [] { const char* e = getenv("MORL_MN_MULTICAST"); return e && e[0] == '1'; }();
-        if (mc_env && n_tiles == 2 && NB == 256) {
-            if (!attr_set_mc) {
-                cudaFuncSetAttribute(gemm_planes_mn_kernel<kFmt, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                attr_set_mc = true;
-            }
-            cudaLaunchConfig_t cfg;
-            memset(&cfg, 0, sizeof(cfg));
-            cfg.gridDim = dim3(n_tiles * S);
-            cfg.blockDim = dim3(192);
-            cfg.dynamicSmemBytes = smem;
-            cfg.stream = st;
-            cudaLaunchAttribute attr[2];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = 2;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[1].val.programmaticStreamSerializationAllowed = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = pdl_enabled() ? 2 : 1;
-            cudaLaunchKernelEx(&cfg, gemm_planes_mn_kernel<kFmt, 1>, tmA, tmB, g);
-        } else {
-            launch_k(gemm_planes_mn_kernel<kFmt, 0>, dim3(n_tiles * S), dim3(192), smem, st, tmA, tmB, g);
-        }
-    });
-    rc = check_launch("morl_gemm_planes_mn_f32");
+    MORL_REQUIRE(aligned16(workspace), MORL_ERR_ALIGN, "morl_gemm_planes_mn_f32: workspace must be 16-byte aligned");
+    MnMulti mj;
+    memset(&mj, 0, sizeof(mj));
+    mj.M = M;
+    const MorlMnJob q = {g_planes, g_plane_stride, g_scale, h_planes, h_plane_stride, h_scale, out, colsum_out, ldg, g_cols, ldh, h_cols, ld_out};
+    float* ws = static_cast<float*>(workspace);
+    int red_blocks = 0;
+    int rc = mn_add_job("morl_gemm_planes_mn_f32", fmt, q, mj, ws, red_blocks);
     if (rc) return rc;
-    const int total = g_cols * h_cols;
-    const int main_blocks = (total + 31) / 32, vec_blocks = colsum_out ? (g_cols + 31) / 32 : 0;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    rc = mn_launch("morl_gemm_planes_mn_f32", fmt, mj, st);
+    if (rc) return rc;
     if (!transpose_out && h_cols % 4 == 0 && ld_out % 4 == 0 && aligned16(out)) {
-        const int mb4 = (total / 4 + 31) / 32;
-        launch_k(reduce_partials_vec4_kernel, dim3(mb4 + vec_blocks), dim3(dim3(32, 8)), 0, st, g.partial, S, n_tiles * 128, NB, g_cols, h_cols, out, ld_out, mb4,
-                                                                              g.colsum_partial, colsum_out, g_scale, h_scale);
+        launch_k(reduce_partials_vec4_multi_kernel, dim3(red_blocks), dim3(32, 8), 0, st, mj);
         return check_launch("morl_gemm_planes_mn_f32(reduce)");
     }
-    launch_k(reduce_partials_kernel, dim3(main_blocks + vec_blocks), dim3(dim3(32, 8)), 0, st, g.partial, S, n_tiles * 128, NB, g_cols, h_cols, transpose_out, out, ld_out,
-                                                                             main_blocks, g.colsum_partial, colsum_out, g_scale, h_scale);
+    // transposed or odd-width output: the scalar reduction of the same [S][g_cols][NB] partials, summed in the same order
+    const MnJobArgs& a = mj.job[0];
+    const int main_blocks = (g_cols * h_cols + 31) / 32, vec_blocks = colsum_out ? (g_cols + 31) / 32 : 0;
+    launch_k(reduce_partials_kernel, dim3(main_blocks + vec_blocks), dim3(32, 8), 0, st, a.partial, a.S, g_cols, a.NB, g_cols, h_cols, transpose_out, out,
+             ld_out, main_blocks, a.colsum_partial, colsum_out, g_scale, h_scale);
     return check_launch("morl_gemm_planes_mn_f32(reduce)");
 }
 
@@ -1949,56 +1788,19 @@ extern "C" int morl_gemm_planes_mn_multi_f32(int fmt, const MorlMnJob* jobs, int
     MORL_REQUIRE(aligned16(workspace), MORL_ERR_ALIGN, "morl_gemm_planes_mn_multi_f32: workspace must be 16-byte aligned");
     MnMulti mj;  // (host staging; copied into the kernel parameters by the launches)
     memset(&mj, 0, sizeof(mj));
-    mj.n_jobs = n_jobs;
     mj.M = M;
     float* ws = static_cast<float*>(workspace);
-    int units = 0, red_blocks = 0;
+    int red_blocks = 0;
     for (int i = 0; i < n_jobs; ++i) {
         const MorlMnJob& q = jobs[i];
-        MORL_REQUIRE(q.g_planes && q.h_planes && q.out, MORL_ERR_NULL, "morl_gemm_planes_mn_multi_f32: job %d has a NULL pointer", i);
-        MORL_REQUIRE(q.g_cols > 0 && q.h_cols > 0 && q.ldg % 64 == 0 && q.ldh % 64 == 0 && q.ldh <= 256 && q.g_cols <= q.ldg && q.h_cols <= q.ldh,
-                     MORL_ERR_SHAPE, "morl_gemm_planes_mn_multi_f32: job %d: bad shape g_cols=%d ldg=%d h_cols=%d ldh=%d (ld multiples of 64, ldh <= 256)", i,
-                     q.g_cols, q.ldg, q.h_cols, q.ldh);
-        const int n_tiles = (q.g_cols + 127) / 128;
-        MORL_REQUIRE(n_tiles * 128 <= q.ldg || q.ldg % 128 == 0 || n_tiles * 128 - q.ldg <= 64, MORL_ERR_UNSUPPORTED,
-                     "morl_gemm_planes_mn_multi_f32: job %d: ldg=%d", i, q.ldg);
+        const int rc = mn_add_job("morl_gemm_planes_mn_multi_f32", fmt, q, mj, ws, red_blocks);
+        if (rc) return rc;
         // the reduction stores four consecutive columns per thread
         MORL_REQUIRE(q.h_cols % 4 == 0 && q.ld_out >= q.h_cols && q.ld_out % 4 == 0 && aligned16(q.out), MORL_ERR_UNSUPPORTED,
                      "morl_gemm_planes_mn_multi_f32: job %d: needs h_cols %% 4 == 0, ld_out %% 4 == 0 (>= h_cols) and a 16-byte aligned output", i);
-        MnJobArgs& a = mj.job[i];
-        mn_split(M, n_tiles, a.S, a.rows_per_split);
-        a.n_tiles = n_tiles;
-        a.NB = (q.h_cols + 63) / 64 * 64;
-        a.g_cols = q.g_cols; a.h_cols = q.h_cols; a.ld_out = q.ld_out;
-        a.unit0 = units;
-        units += n_tiles * a.S;
-        a.partial = ws;
-        a.colsum_partial = q.colsum_out ? ws + (size_t)a.S * q.g_cols * a.NB : nullptr;
-        ws += mn_multi_job_floats(M, q.g_cols, q.h_cols);
-        a.out = q.out; a.colsum_out = q.colsum_out; a.g_scale = q.g_scale; a.h_scale = q.h_scale;
-        a.red_block0 = red_blocks;
-        a.red_main_blocks = (q.g_cols * q.h_cols / 4 + 31) / 32;
-        red_blocks += a.red_main_blocks + (q.colsum_out ? (q.g_cols + 31) / 32 : 0);
-        int rc = make_plane_map_mn(&mj.tmA[i], fmt, q.g_planes, M, q.ldg, q.g_plane_stride);
-        MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_multi_f32: job %d: cuTensorMapEncodeTiled(G) failed (%d)", i, rc);
-        rc = make_plane_map_mn(&mj.tmB[i], fmt, q.h_planes, M, q.ldh, q.h_plane_stride);
-        MORL_REQUIRE(rc == 0, MORL_ERR_NO_DEVICE, "morl_gemm_planes_mn_multi_f32: job %d: cuTensorMapEncodeTiled(H) failed (%d)", i, rc);
     }
-    mj.n_units = units;
-    int sms = morl_device_sm_count();
-    if (sms <= 0) sms = 148;
-    const int grid = units < sms ? units : sms;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MORL_DISPATCH_FMT(fmt, {
-        constexpr size_t smem = mn_smem_bytes<kFmt>();
-        static bool attr_set = false;
-        if (!attr_set) {
-            cudaFuncSetAttribute(gemm_planes_mn_multi_kernel<kFmt>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            attr_set = true;
-        }
-        launch_k(gemm_planes_mn_multi_kernel<kFmt>, dim3(grid), dim3(kGemmThreads), smem, st, mj);
-    });
-    const int rc = check_launch("morl_gemm_planes_mn_multi_f32");
+    const int rc = mn_launch("morl_gemm_planes_mn_multi_f32", fmt, mj, st);
     if (rc) return rc;
     launch_k(reduce_partials_vec4_multi_kernel, dim3(red_blocks), dim3(32, 8), 0, st, mj);
     return check_launch("morl_gemm_planes_mn_multi_f32(reduce)");

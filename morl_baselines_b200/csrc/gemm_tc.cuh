@@ -98,21 +98,6 @@ __device__ __forceinline__ void tc_mma_bf16_pair(uint32_t tmem_d, uint64_t adesc
         "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// one box for several CTAs of the cluster (mask: bit r = CTA rank r): written at the same shared-memory offset in each of them, completing on the
-// mbarrier at the same offset in each of them
-__device__ __forceinline__ void tma_load_3d_multicast(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(
-            g_smem_u32(dst)),
-        "l"(map), "r"(g_smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-        : "memory");
-}
-// commit of a CTA's own (cta_group::1) MMAs, arriving on the barrier at this offset in BOTH CTAs of a 2-CTA cluster
-__device__ __forceinline__ void tc_commit_mc(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(g_smem_u32(bar)),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_commit(uint64_t* bar) {

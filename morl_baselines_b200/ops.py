@@ -657,8 +657,8 @@ def gemm_mn_workspace(M: int, g_cols: int, h_cols: int, device) -> th.Tensor:
 def gemm_planes_mn(g_planes: th.Tensor, g_cols: int, h_planes: th.Tensor, h_cols: int, transpose_out: bool = False,
                    out: Optional[th.Tensor] = None, workspace: Optional[th.Tensor] = None, colsum: Optional[th.Tensor] = None,
                    g_scale: Optional[th.Tensor] = None, h_scale: Optional[th.Tensor] = None) -> th.Tensor:
-    """out[n, k] = sum_m G[m, n] H[m, k] (weight gradient; reduction over the rows) from plane tensors [P, M, ld] (scales removed).
-    ``colsum`` ([g_cols] fp32, optional) additionally receives sum_m G[m, n] (the bias gradient) from the same pass."""
+    """out[n, k] = sum_m G[m, n] H[m, k] (weight gradient; reduction over the rows) from plane tensors [P, M, ld] (scales removed), as a
+    one-job launch of the :class:`GemmMnMulti` kernel.  ``colsum`` ([g_cols] fp32, optional) also receives sum_m G[m, n] (the bias gradient)."""
     fmt = fmt_of(g_planes)
     _, M, ldg = g_planes.shape
     _, M2, ldh = h_planes.shape
@@ -678,8 +678,8 @@ def gemm_planes_mn(g_planes: th.Tensor, g_cols: int, h_planes: th.Tensor, h_cols
 class GemmMnMulti:
     """Static plan of several weight-gradient products over the same rows in ONE persistent launch plus one reduction
     (morl_gemm_planes_mn_multi_f32): each entry of ``jobs`` is ``(g_planes, g_cols, h_planes, h_cols, out, colsum, g_scale, h_scale)``
-    with the meaning of :func:`gemm_planes_mn` (``colsum`` and the scales may be None; ``out`` is [g_cols, h_cols], not transposed).  Every
-    output is bit-identical to the per-product :func:`gemm_planes_mn` call.  The job table and the workspace are built once; a call is two launches."""
+    with the meaning of :func:`gemm_planes_mn` (``colsum`` and the scales may be None; ``out`` is [g_cols, h_cols], not transposed).  No output
+    depends on the other jobs: each is bit-identical to :func:`gemm_planes_mn` of that job alone.  Table and workspace are built once; a call is two launches."""
 
     def __init__(self, jobs):
         if not 1 <= len(jobs) <= _lib.MN_MAX_JOBS:

@@ -47,7 +47,6 @@ from . import ops
 _SNAKE = os.environ.get("MORL_TC_SNAKE", "1") == "1"          # alternate the GEMM tile order between chained layers
 _CHAIN = os.environ.get("MORL_GEMM_CHAIN", "1") == "1"        # hidden layers 2.. of a pass as ONE chained launch (+10 % on the update; =0: one launch per layer)
 _CHAIN_BWD = os.environ.get("MORL_GEMM_CHAIN_BWD", "1") == "1"  # ... and the 256-wide dX products of the backward pass (+2.7 %; =0: per-layer launches)
-_MN_MULTI = os.environ.get("MORL_MN_MULTI", "1") == "1"          # ... and all weight-gradient products of it as ONE launch + one reduction (=0: per layer)
 _NARROW_HEAD = os.environ.get("MORL_NARROW_HEAD", "1") == "1"  # output layer through morl_qhead_gemm_f32 (19.7 us against 26 us in the update; =0: general kernel)
 _DEFAULT_FMT = ops.FMT_BF16X3 if os.environ.get("MORL_TC_FMT", "f16x2") == "bf16x3" else ops.FMT_F16X2
 
@@ -284,27 +283,25 @@ class TCPairMlp:
         grads[0], grads[1] = ops.pair_layer1_grad(dU, dV, feats, wset, dW1=grads[0], db1=grads[1], workspace=self.ws_l1)
         return grads
 
-
-def _backward_chained(self, feats, wset, G, grads, after_gemms):
-    """Backward with the 256-wide dX products as ONE chained launch: G_{n-2} from the (narrow) output layer as before, then
-    G_{k-1} = (G_k . W_k) * relu'(H_{k-1}) for k = n-2 .. 1 in one persistent kernel (each G_k in its own buffer: the weight-gradient
-    products read them afterwards), then the n-1 weight-gradient GEMMs -- one multi-job launch (ops.GemmMnMulti), or per layer with
-    MORL_MN_MULTI=0 (the output layer's before the chain)."""
-    n = len(self.lin)
-    dev = G.device
-    if self._gchain is None:
-        M, hid = self.B * self.W, self.lin[1].in_features
-        self._gbufs = [ops.empty_planes(self.fmt, M, hid, dev) for _ in range(n - 1)]  # dL/d(output of lin[n-2]), ..., dL/d(output of lin[0])
-        # chain input = the planes of dL/dQ (ld_last wide: the first job reduces over ld_last columns only), outputs the n - 1 hidden gradients
-        ks = list(range(n - 1, 0, -1))  # layers whose dX product is in the chain: the narrow output layer first
-        self._gchain = ops.GemmChain([[self.g_last] + self._gbufs], [[self.wtp[k - 1] for k in ks]], None, [[self.s_w[k - 1] for k in ks]], None,
-                                     act_scale=self.s_g, relu=False, bits_in=[[self.hbits[k - 1] for k in ks]], k_first=self.ld_last)
-    for k in range(1, n):
-        if grads[2 * k] is None:
-            grads[2 * k] = th.empty((self.lin[k].out_features, self.lin[k].in_features), device=dev, dtype=th.float32)
-        if grads[2 * k + 1] is None:
-            grads[2 * k + 1] = th.empty(self.lin[k].out_features, device=dev, dtype=th.float32)
-    if _MN_MULTI and n - 1 <= ops._lib.MN_MAX_JOBS:
+    def _backward_chained(self, feats, wset, G, grads, after_gemms):
+        """Backward with the 256-wide dX products as ONE chained launch: G_{n-2} from the (narrow) output layer as before, then
+        G_{k-1} = (G_k . W_k) * relu'(H_{k-1}) for k = n-2 .. 1 in one persistent kernel (each G_k in its own buffer: the weight-gradient
+        products read them afterwards), then the n-1 weight-gradient products as multi-job launches (ops.GemmMnMulti), at most
+        MN_MAX_JOBS products per launch."""
+        n = len(self.lin)
+        dev = G.device
+        if self._gchain is None:
+            M, hid = self.B * self.W, self.lin[1].in_features
+            self._gbufs = [ops.empty_planes(self.fmt, M, hid, dev) for _ in range(n - 1)]  # dL/d(output of lin[n-2]), ..., dL/d(output of lin[0])
+            # chain input = the planes of dL/dQ (ld_last wide: the first job reduces over ld_last columns only), outputs the n - 1 hidden gradients
+            ks = list(range(n - 1, 0, -1))  # layers whose dX product is in the chain: the narrow output layer first
+            self._gchain = ops.GemmChain([[self.g_last] + self._gbufs], [[self.wtp[k - 1] for k in ks]], None, [[self.s_w[k - 1] for k in ks]], None,
+                                         act_scale=self.s_g, relu=False, bits_in=[[self.hbits[k - 1] for k in ks]], k_first=self.ld_last)
+        for k in range(1, n):
+            if grads[2 * k] is None:
+                grads[2 * k] = th.empty((self.lin[k].out_features, self.lin[k].in_features), device=dev, dtype=th.float32)
+            if grads[2 * k + 1] is None:
+                grads[2 * k + 1] = th.empty(self.lin[k].out_features, device=dev, dtype=th.float32)
         self._gchain()  # all n - 1 dX products (the narrow one of the output layer included) in one launch
         key = tuple(grads[i].data_ptr() for i in range(2, 2 * n))
         if self._mn_multi is None or self._mn_multi[0] != key:
@@ -314,31 +311,19 @@ def _backward_chained(self, feats, wset, G, grads, after_gemms):
                      self.s_act) for k in range(1, n - 1)]
             jobs.append((G, self.lin[n - 1].out_features, self.h[n - 2], self.lin[n - 1].in_features, grads[2 * (n - 1)], grads[2 * (n - 1) + 1], self.s_g,
                          self.s_act))
-            self._mn_multi = (key, ops.GemmMnMulti(jobs))
-        self._mn_multi[1]()
+            per = ops._lib.MN_MAX_JOBS
+            self._mn_multi = (key, [ops.GemmMnMulti(jobs[i:i + per]) for i in range(0, len(jobs), per)])
+        for plan in self._mn_multi[1]:
+            plan()
         return self._backward_tail(feats, wset, grads, after_gemms)
-    last = self.lin[n - 1]
-    grads[2 * (n - 1)] = ops.gemm_planes_mn(G, last.out_features, self.h[n - 2], last.in_features, out=grads[2 * (n - 1)], workspace=self.ws_mn,
-                                            colsum=grads[2 * (n - 1) + 1], g_scale=self.s_g, h_scale=self.s_act)
-    self._gchain()  # all n - 1 dX products (the narrow one of the output layer included) in one launch
-    for i, k in enumerate(range(n - 2, 0, -1)):  # dW_k = (dL/dh_k)^T H_{k-1}: dL/dh_k is _gbufs[i]
-        l = self.lin[k]
-        grads[2 * k] = ops.gemm_planes_mn(self._gbufs[i], l.out_features, self.h[k - 1], l.in_features, out=grads[2 * k], workspace=self.ws_mn,
-                                          colsum=grads[2 * k + 1], g_scale=self.s_g, h_scale=self.s_act)
-    return self._backward_tail(feats, wset, grads, after_gemms)
 
-
-def _backward_tail(self, feats, wset, grads, after_gemms):
-    """After the last tensor-core GEMM of the chained backward: fork the side work, then the layer-1 gradients."""
-    if after_gemms is not None:
-        after_gemms()
-    dU, dV = ops.pairs_grad_reduce(self._gbufs[len(self.lin) - 2], self.B, self.W, workspace=self.ws_red, dU=self.dU, dV=self.dV, scale=self.s_g)
-    grads[0], grads[1] = ops.pair_layer1_grad(dU, dV, feats, wset, dW1=grads[0], db1=grads[1], workspace=self.ws_l1)
-    return grads
-
-
-TCPairMlp._backward_chained = _backward_chained
-TCPairMlp._backward_tail = _backward_tail
+    def _backward_tail(self, feats, wset, grads, after_gemms):
+        """After the last tensor-core GEMM of the chained backward: fork the side work, then the layer-1 gradients."""
+        if after_gemms is not None:
+            after_gemms()
+        dU, dV = ops.pairs_grad_reduce(self._gbufs[len(self.lin) - 2], self.B, self.W, workspace=self.ws_red, dU=self.dU, dV=self.dV, scale=self.s_g)
+        grads[0], grads[1] = ops.pair_layer1_grad(dU, dV, feats, wset, dW1=grads[0], db1=grads[1], workspace=self.ws_l1)
+        return grads
 
 
 class TCPairMlpFn(th.autograd.Function):

@@ -1,5 +1,6 @@
 """GPU tests of the multi-job weight-gradient launch (ops.GemmMnMulti, csrc/gemm_planes.cu: gemm_planes_mn_multi_kernel): every dW and
-db must be BIT-identical to the per-product ops.gemm_planes_mn call (same split boundaries, MMA order and reduction order)."""
+db must be BIT-identical to the one-job ops.gemm_planes_mn call on that product alone, i.e. dealing the units of several jobs together
+changes no bit.  tests/test_gemm_mn_golden_gpu.py pins the one-job results to the recorded outputs of the former per-layer kernel."""
 
 import pytest
 import torch as th

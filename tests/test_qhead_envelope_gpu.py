@@ -183,13 +183,28 @@ def test_narrow_head_gemm_equals_general_gemm(cuda, M, N, K):
 def test_chained_passes_equal_per_layer_passes(cuda):
     """TCPairMlp forward / backward with the hidden layers as chained launches (forward chain, dX chain) == the per-layer launches, bit for
     bit: Q, every gradient tensor."""
+    _chained_equals_per_layer(cuda, n_hidden=4)
+
+
+def test_chained_backward_of_a_deep_net_equals_per_layer_passes(cuda):
+    """Six weight-gradient products: more than one multi-job launch takes them (MN_MAX_JOBS per launch), still bit-identical."""
+    from morl_baselines_b200 import _lib
+
+    assert 6 > _lib.MN_MAX_JOBS
+    _chained_equals_per_layer(cuda, n_hidden=6)
+
+
+def _chained_equals_per_layer(cuda, n_hidden):
     from torch import nn
 
     from morl_baselines_b200 import ops, tc_mlp
 
     th.manual_seed(3)
     B, W, F, D, H, OUT = 64, 8, 12, 3, 256, 12
-    net = nn.Sequential(nn.Linear(F + D, H), nn.ReLU(), nn.Linear(H, H), nn.ReLU(), nn.Linear(H, H), nn.ReLU(), nn.Linear(H, H), nn.ReLU(), nn.Linear(H, OUT)).to(cuda)
+    layers = [nn.Linear(F + D, H), nn.ReLU()]  # (built in this order: the seeded weights of every layer stay those of n_hidden = 4)
+    for _ in range(n_hidden - 1):
+        layers += [nn.Linear(H, H), nn.ReLU()]
+    net = nn.Sequential(*layers, nn.Linear(H, OUT)).to(cuda)
     feats, wset = th.randn(B, F, device=cuda), th.rand(W, D, device=cuda)
     dq = th.randn(B * W, OUT, device=cuda) * 1e-3
     results = []
